@@ -12,7 +12,7 @@ process).  Keys of the JSON line:
   value      tokens/s with everything resident in HBM: K / (CUDA-event time around the K timed evals' kernels on the library stream),
              whole job over all ranks (max over ranks of the time)
   e2e        tokens/s through the reference-facing API -- fastllama_b200.Model.generate() on the drop-in pyfastllama.so (the
-             reference's unchanged bridge): wall clock around the call, which per step copies the token id + position host->device
+             llama_* C ABI over libggml_b200): wall clock around the call, which per step copies the token id + position host->device
              (pinned) and the logits + embeddings row device->host (pinned staging)
   roofline   dominant kernel = k_decode_token, the persistent kernel that runs the whole decode step (one launch per token, reads every
              quantised weight once): algorithmic bytes per launch / mean launch duration (CUDA events on the launching stream),
@@ -293,13 +293,34 @@ class Backend:
 GREEDY = dict(temp=0.0, top_k=1, top_p=1.0, repeat_penalty=1.0)
 
 
+def _synth_vocab():
+    from fastllama_b200.ggjt import vocab_entries
+
+    return {tok.decode(): i for i, (tok, _) in enumerate(vocab_entries(32000))}
+
+
+SYNTH_VOCAB = _synth_vocab()          # text -> id of the synthetic model's vocabulary: every token streams as its own text
+
+
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: what the timed path computed, as DIR/<name>.npy (logits float32, token ids float64)."""
+    if not out_dir:
+        return
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float32 if name == "logits" else np.float64))
+
+
 def timed_decode(be: Backend, m, steps: int, dist=None, local_rank=0, sample_clocks=True):
     """K decode steps through Model.generate: device time (CUDA events around each eval's launches, summed by the library), wall
     clock, launches.  The streaming callback only counts: nothing but the reference-facing call sits in the timed region."""
-    count = [0]
+    count, streamed = [0], []
 
-    def on_token(_s):
+    def on_token(s):
         count[0] += 1
+        streamed.append(s)
 
     if dist:
         dist.barrier()
@@ -321,7 +342,7 @@ def timed_decode(be: Backend, m, steps: int, dist=None, local_rank=0, sample_clo
         sampler.join(timeout=2)
     hp = be.host_profile(reset=True)
     n_evals = int(s1.n_evals - s0.n_evals)
-    return {"tokens": count[0], "evals": n_evals, "device_s": (s1.total_device_us - s0.total_device_us) * 1e-6, "wall_s": t1 - t0, "launches": int(launches),
+    return {"tokens": count[0], "token_ids": [SYNTH_VOCAB.get(t, -1) for t in streamed], "evals": n_evals, "device_s": (s1.total_device_us - s0.total_device_us) * 1e-6, "wall_s": t1 - t0, "launches": int(launches),
             "clocks": sampler.summary() if sampler else None,
             "host_us_per_step": ({"graph_match": hp[1] / hp[0], "match_scalars_launch_issue": hp[2] / hp[0], "device_wait_and_result_copies": hp[3] / hp[0],
                                   "caller_between_steps(sampling, graph build, callback)": hp[4] / hp[0]} if hp[0] else None)}
@@ -362,21 +383,28 @@ def committed_traffic():
         return None, None
 
 
-def ingest_run(be: Backend, path: str, size: str, wtype_name: str, peaks, peak_src, batches: int = 2):
-    """Prompt ingest with n_batch = 128: the prompt is batches*128 + 1 tokens, so ingest() evaluates `batches` full 128-token
-    chunks (the last chunk, one token, is left to the first generate(); reference lib/bridge.cpp:213-232)."""
+def ingest_run(be: Backend, path: str, size: str, wtype_name: str, peaks, peak_src, steps: int = 2):
+    """Prompt ingest with n_batch = 128: `steps` timed evals of 128 prompt tokens.  The 512-token context holds three of them, so they
+    run in groups of at most three, each group one prompt of group*128 + 1 tokens on a reset model (ingest() evaluates the full
+    128-token chunks; the last chunk, one token, is left to the first generate(); reference lib/bridge.cpp:213-232)."""
     m = be.model(path, n_batch=128)
     warm = _long_prompt(128 + 1 - 2)
     assert m.ingest(warm)                                  # uploads the weights, builds the N = 128 path once (untimed)
     m.generate(lambda s: None, num_tokens=1, **GREEDY)
-    assert m.reset()
     be.fl.check(be.fl.lib.fl_sync())
     s0 = be.stats()
     l0 = be.fl.lib.fl_launch_count()
-    t0 = time.perf_counter()
-    assert m.ingest(_long_prompt(batches * 128 + 1 - 2, salt=3))
-    be.fl.check(be.fl.lib.fl_sync())
-    t1 = time.perf_counter()
+    wall = 0.0
+    left = steps
+    while left > 0:
+        batches = min(3, left)
+        assert m.reset()
+        t0 = time.perf_counter()
+        assert m.ingest(_long_prompt(batches * 128 + 1 - 2, salt=3))
+        be.fl.check(be.fl.lib.fl_sync())
+        wall += time.perf_counter() - t0
+        left -= batches
+    last_logits = m.get_logits_array()                     # the last timed eval's logits (its last token)
     s1 = be.stats()
     evals = int(s1.n_evals - s0.n_evals)
     dev_s = (s1.total_device_us - s0.total_device_us) * 1e-6
@@ -389,7 +417,7 @@ def ingest_run(be: Backend, path: str, size: str, wtype_name: str, peaks, peak_s
     algo = ALGO_BYTES_PER_TOKEN.get((size, wtype_name))
     res = {"metric": f"prompt tokens/sec LLaMA-{size} {wtype_name} ingest (n_batch=128)", "value": n_tok / dev_s if dev_s else 0.0, "unit": "tokens/s", "steps": evals,
            "ms_per_step": per_eval * 1e3, "config": {"workload": f"LLaMA-{size} {wtype_name} prompt ingest, n_batch=128, {evals} evals of 128 tokens at n_past 0..{n_tok - 128}, n_ctx=512"},
-           "e2e": {"value": n_tok / (t1 - t0), "unit": "tokens/s", "h2d_bytes_per_step": 128 * 4, "d2h_bytes_per_step": 32000 * 4 + 4 * {"7B": 4096, "13B": 5120, "65B": 8192}[size]},
+           "e2e": {"value": n_tok / wall, "unit": "tokens/s", "h2d_bytes_per_step": 128 * 4, "d2h_bytes_per_step": 32000 * 4 + 4 * {"7B": 4096, "13B": 5120, "65B": 8192}[size]},
            "gpu_launches": launches,
            "roofline": {"bound": "tensor", "achieved": tf, "peak": peak_t, "unit": "TFLOP/s", "frac": tf / peak_t, "traffic": None,
                         "kernel": "k_mul_mat_q_umma (tcgen05.mma kind::i8, one MMA per quant block into TMEM; exact fp32 block scaling on the CUDA cores) -- the whole eval "
@@ -406,7 +434,7 @@ def ingest_run(be: Backend, path: str, size: str, wtype_name: str, peaks, peak_s
             # generate(1) so that the timed steps are all N = 1
             assert m.ingest(_long_prompt(464 - (batches * 128 + 16 + 1) - 2, salt=5))
             m.generate(lambda s: None, num_tokens=1, **GREEDY)
-        r = timed_decode(be, m, 16, sample_clocks=False)
+        r = timed_decode(be, m, 16, sample_clocks=False)       # 16 steps: what the 512-token context holds after these prompts
         if r["evals"]:
             cur = r
         if cur and algo:
@@ -422,6 +450,7 @@ def ingest_run(be: Backend, path: str, size: str, wtype_name: str, peaks, peak_s
                                  "steps": cur["evals"], "ms_per_step": 1e3 * cur["device_s"] / cur["evals"], "e2e": {"value": cur["tokens"] / cur["wall_s"], "unit": "tokens/s"},
                                  "config": {"workload": f"LLaMA-{size} {wtype_name} greedy decode at n_past ~{n_past_mid} of n_ctx 512"}, "roofline": rl})
     m.close()
+    res["last_logits"] = last_logits
     return res, extra_decode
 
 
@@ -442,6 +471,7 @@ def decode_run(be: Backend, path, size, wtype_name, steps, warmup, peaks, peak_s
         logits.append(m.get_logits_array())
     m.generate(lambda s: None, num_tokens=max(warmup - len(toks), 3), **GREEDY)       # >= 3 untimed warm-up steps on the graph-replay path
     r = timed_decode(be, m, steps, dist=dist, local_rank=local_rank)
+    r["last_logits"] = m.get_logits_array()                      # what the caller holds after the last timed step
     mode = int(be.ggml.ggml_b200_decode_mode())
     m.close()
     return r, mode, toks, (np.stack(logits) if logits else None)
@@ -497,6 +527,9 @@ def main():
     ap.add_argument("--parity-tokens", type=int, default=32)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the timed path computed to DIR: logits.npy (float32, the last timed eval's logits) and, for decode, "
+                         "tokens.npy (float64, the token ids the timed steps produced), to compare two builds output for output")
     ap.add_argument("--_gen", nargs=2, default=None, help=argparse.SUPPRESS)
     ap.add_argument("--_ref-worker", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
@@ -580,11 +613,12 @@ def main():
 
     if args.mode == "ingest":
         assert world == 1, "--mode ingest is a single-GPU measurement"
-        res, extra_decode = ingest_run(be, path, args.size, args.wtype, peaks, peak_src, batches=max(1, min(3, args.steps)))
+        res, extra_decode = ingest_run(be, path, args.size, args.wtype, peaks, peak_src, steps=args.steps)
         res.update({"n_gpus": 1, "warmup": 1, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u8", "data": "synthetic"})
         res["config"] = config
         res["device"] = be.props["name"]
         res["extra"] = extra_decode
+        dump_outputs(args.dump_outputs, logits=res.pop("last_logits"))
         emit(res)
         return
 
@@ -593,7 +627,11 @@ def main():
     cpu_baseline, parity = None, None
     ref_tokens, ref_logits = [], None
     parity_n = args.parity_tokens if headline else 0
-    if rank == 0 and world == 1 and not args.no_cpu_baseline:
+    from oracle.pyoracle import REF_PYFASTLLAMA_SO
+
+    if rank == 0 and world == 1 and not args.no_cpu_baseline and not os.path.exists(REF_PYFASTLLAMA_SO):
+        log("[bench] cpu_baseline and parity skipped: the reference's CPU library (oracle/_ref) is not built here")
+    elif rank == 0 and world == 1 and not args.no_cpu_baseline:
         import numpy as np
 
         with tempfile.TemporaryDirectory() as td:
@@ -610,6 +648,8 @@ def main():
     if n_tok < args.steps:
         log(f"[bench] rank {rank}: generation stopped after {n_tok} of {args.steps} tokens (EOS); rates use the tokens produced")
     wall, device_s = r["wall_s"], r["device_s"]
+    if rank == 0:
+        dump_outputs(args.dump_outputs, logits=r["last_logits"], tokens=r["token_ids"])
     tok_file = os.path.join(bench_dir(), f"fastllama_b200_parity_{args.size}_{args.wtype}_n1.json")
     if world == 1 and our_tokens:
         if ref_tokens:
@@ -674,7 +714,7 @@ def main():
         "scaling": "weak" if (world > 1 and not tp) else "strong",
         "vs_baseline": None, "dtype": "u8", "data": "synthetic", "config": config,
         "e2e": {"value": e2e, "unit": "tokens/s", "h2d_bytes_per_step": 8, "d2h_bytes_per_step": 32000 * 4 + n_embd_model * 4,
-                "api": "fastllama_b200.Model.generate -> pyfastllama.so (reference bridge, unchanged) -> libggml_b200 -> libfl_cuda",
+                "api": "fastllama_b200.Model.generate -> pyfastllama.so (llama_* C ABI) -> libggml_b200 -> libfl_cuda",
                 "host_us_per_step": r["host_us_per_step"]},
         "gpu_launches": r["launches"], "roofline": rl, "clocks": r["clocks"], "parallelism_detail": par_detail, "device": be.props["name"],
     }
@@ -689,7 +729,8 @@ def main():
     if headline and world == 1 and not args.no_extras and not os.environ.get("FASTLLAMA_BENCH_NO_EXTRAS"):
         extra = []
         try:
-            res, extra_decode = ingest_run(be, path, "7B", "q4_0", peaks, peak_src, batches=2)
+            res, extra_decode = ingest_run(be, path, "7B", "q4_0", peaks, peak_src, steps=2)
+            res.pop("last_logits")
             extra.append(res)
             extra.extend(extra_decode)
         except Exception as e:                                     # an extra never takes the headline line down

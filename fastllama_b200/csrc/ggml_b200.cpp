@@ -656,6 +656,25 @@ static void drop_external_mirrors() {
     if (any) packed_shards_clear();
     g_last_mirror = -1;
 }
+// Records of arenas that no open context covers any more.  Their buffers may have been freed, and foreign memory placed at those
+// addresses later (a model file mapped where an earlier model's arena was) would otherwise resolve to the dead record: a stale
+// device copy, or an upload that reads the old arena's length past the new memory.  Every arena in use re-registers at ggml_init.
+static void drop_closed_arenas() {
+    bool any = false;
+    for (auto &m : g_mirrors) {
+        if (!m.alive || m.kind != MK_ARENA) continue;
+        bool open = false;
+        for (const auto &slot : g_slots) open = open || (slot.used && slot.ctx.mem_buffer == m.host);
+        if (open) continue;
+        if (!any && fl_is_initialized()) fl_sync();
+        any = true;
+        drop_mirror(m);
+        m.alive = false;
+        m.uploaded = 0;
+    }
+    if (any) packed_shards_clear();
+    g_last_mirror = -1;
+}
 static void mirrors_on_ctx_init(ggml_context *ctx) {
     // an arena re-created over the same buffer (Model::eval does this every call) re-uses its mirror
     int found = -1;
@@ -677,7 +696,10 @@ static void mirrors_on_ctx_init(ggml_context *ctx) {
     // (include/tensor/mem_context.hpp:12-16, lib/llama.cpp:213-258).  MK_EXTERNAL mirrors are keyed by host address only, and a
     // new mapping may land on the addresses of an earlier model's: everything registered for earlier mappings is stale now.
     // (A model that is still alive simply re-registers and re-uploads its tensors on next use.)
-    if (ctx->no_alloc) drop_external_mirrors();
+    if (ctx->no_alloc) {
+        drop_external_mirrors();
+        drop_closed_arenas();
+    }
 }
 static void mirrors_on_ctx_free(ggml_context *) {}   // the arena (and its device mirror) outlives the context slot
 static void mirrors_note_alloc(ggml_context *ctx, size_t end) {
@@ -780,9 +802,8 @@ extern "C" void ggml_b200_release_all(void) {
         if (m.device_dirty) { m.device_dirty = false; g_dirty_arenas.fetch_sub(1, std::memory_order_release); }
         if (m.kind != MK_ARENA) m.alive = false;
     }
-    // arenas whose host buffer is gone would never be matched again: forget all records (a live arena re-registers at its next ggml_init,
-    // and a context that is still open keeps working because mirror lookups are by address)
-    g_last_mirror = -1;
+    // an arena whose context is still open keeps its record (lookups are by address); the others are forgotten
+    drop_closed_arenas();
 }
 // how the last single-token eval ran: 0 = node-by-node executor, 1 = fused plan with one kernel per matrix group,
 // 2 = fused plan as one persistent kernel per token (fl_token_kernel.cu)

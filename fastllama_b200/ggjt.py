@@ -130,3 +130,23 @@ def write_synthetic_gpu(path, size="7B", wtype=Q4_0, seed=0, std=0.02, n_vocab=3
     finally:
         fl.free(d_f32)
         fl.free(d_q)
+
+
+GGLA_MAGIC = 0x67676C61
+
+
+def write_lora(path: str, factors: dict, r: int, alpha: int) -> int:
+    """LoRA adapter file ('ggla' v1): u8 cached (0: factors), u32 r, u32 alpha, then per adapted weight W the f32 tensors
+    "<W>.loraA" (ne = r, K; already scaled by alpha / r) and "<W>.loraB" (ne = r, M), records laid out as in write_ggjt.
+    `factors` maps W's name to (A[K, r], B[M, r]) float32 arrays."""
+    with open(path, "wb") as f:
+        f.write(struct.pack("<IIBII", GGLA_MAGIC, 1, 0, r, alpha))
+        for name, mats in factors.items():
+            for tag, m in zip("AB", mats):
+                m = np.ascontiguousarray(m, dtype=np.float32)
+                nm = f"{name}.lora{tag}".encode()
+                f.write(struct.pack("<iiiii", 2, len(nm), F32, m.shape[1], m.shape[0]))
+                f.write(nm)
+                f.write(b"\0" * (-f.tell() & 31))
+                f.write(m.tobytes())
+        return f.tell()

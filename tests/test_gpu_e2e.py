@@ -1,7 +1,7 @@
-"""GPU: end to end through the product boundary B2.  The same prompt is run through
-  * the reference product library (oracle/_ref/pyfastllama_ref.so: reference bridge + reference ggml, CPU)
-  * the drop-in pyfastllama.so of this repo (the reference's UNCHANGED bridge/llama.cpp over libggml_b200)
-via the same Python Model class (fastllama_b200/model.py, mirror of the reference's fastllama.Model).
+"""GPU: end to end through the product boundary B2.  The same prompt is run through the drop-in pyfastllama.so of this repo
+(llama_* C ABI over libggml_b200) via the Python Model class (fastllama_b200/model.py, mirror of the reference's fastllama.Model)
+and compared with what the reference product library (reference bridge + reference ggml, CPU) produced on the same seeded model
+file: tests/golden/model_e2e_toy.npz (oracle/gen_golden_model.py).
 
 north_star bar: greedy token-id sequence identical; logits within a stated fp tolerance.  The tolerance here is ZERO: the logits after
 the prompt and the decode steps carry the reference's bits (every fp32 operation in the reference's order, fl_exact.cuh; the prompt of
@@ -15,10 +15,11 @@ import pytest
 from fastllama_b200.build import lib_path
 from fastllama_b200.ggjt import Q4_0, Q4_1, write_synthetic_numpy
 from fastllama_b200.model import Model, QuietLogger
-from oracle.pyoracle import REF_PYFASTLLAMA_SO, Oracle
+from oracle.pyoracle import Oracle
 
 pytestmark = pytest.mark.gpu
 DROPIN = os.environ.get("FASTLLAMA_TEST_DROPIN", lib_path("pyfastllama.so"))     # tests/mock/build/... for host-logic dry runs
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 PROMPT = "The quick brown fox jumps over the lazy dog. 0123456789"
 
 
@@ -32,16 +33,22 @@ def _run(lib, path, n_batch, n_gen=24):
     return toks, logits
 
 
-@pytest.mark.skipif(not os.path.exists(REF_PYFASTLLAMA_SO), reason="oracle/_ref not built")
+def toy_model(tmp_path, wtype):
+    orc = Oracle()
+    path = str(tmp_path / f"toy{wtype}.bin")
+    write_synthetic_numpy(path, wtype, n_vocab=512, n_embd=256, n_mult=64, n_head=4, n_layer=3, seed=11, std=0.01,
+                          quantize=lambda w, t: orc.quantize_q4(w, t))
+    return path
+
+
 @pytest.mark.parametrize("wtype", [Q4_0, Q4_1])
 @pytest.mark.parametrize("n_batch", [1, 8])
 def test_greedy_tokens_and_logits_match_reference(tmp_path, wtype, n_batch):
-    orc = Oracle()
-    path = str(tmp_path / "toy.bin")
-    write_synthetic_numpy(path, wtype, n_vocab=512, n_embd=256, n_mult=64, n_head=4, n_layer=3, seed=11, std=0.01,
-                          quantize=lambda w, t: orc.quantize_q4(w, t))
+    path = toy_model(tmp_path, wtype)
     assert os.path.exists(DROPIN), "drop-in library not built"
-    ref_toks, ref_logits = _run(REF_PYFASTLLAMA_SO, path, n_batch)
+    golden = np.load(os.path.join(GOLDEN, "model_e2e_toy.npz"))
+    key = f"{'q4_0' if wtype == Q4_0 else 'q4_1'}_b{n_batch}"
+    ref_toks, ref_logits = list(golden[key + "_tokens"]), golden[key + "_logits"]
     our_toks, our_logits = _run(DROPIN, path, n_batch)
     assert len(ref_toks) > 4
     assert our_toks == ref_toks, (our_toks, ref_toks)

@@ -1,33 +1,13 @@
 """GPU: the same save_state / load_state round trip and reference interop as tests/test_state_mock.py, on the real device
 layer (KV cache in HBM, the persistent token kernel writing it)."""
-import os
-
-import numpy as np
 import pytest
 
-from tests.test_state_mock import _run
+from tests.test_state_mock import check_state_interop
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_state_round_trip_and_interop_with_reference_on_gpu(tmp_path):
-    from fastllama_b200.build import LIB_DIR
-    from fastllama_b200.ggjt import Q4_0, write_synthetic_numpy
-    from oracle.pyoracle import REF_PYFASTLLAMA_SO, Oracle
+    from fastllama_b200.build import lib_path
 
-    if not os.path.exists(REF_PYFASTLLAMA_SO):
-        pytest.skip("oracle/_ref not built")
-    orc = Oracle()
-    model = str(tmp_path / "toy.bin")
-    write_synthetic_numpy(model, Q4_0, n_vocab=512, n_embd=256, n_mult=256, n_head=4, n_layer=3, seed=7, std=0.01, quantize=lambda w, t: orc.quantize_q4(w, t))
-    ours_lib = os.path.join(LIB_DIR, "pyfastllama.so")
-
-    ours = _run(tmp_path, "save", ours_lib, model, str(tmp_path / "ours.state"), "ours")
-    assert list(ours["first"]) == list(ours["again"])
-    ref = _run(tmp_path, "save", REF_PYFASTLLAMA_SO, model, str(tmp_path / "ref.state"), "ref")
-    ref_from_ours = _run(tmp_path, "load", REF_PYFASTLLAMA_SO, model, str(tmp_path / "ours.state"), "ref_from_ours")
-    assert list(ref_from_ours["again"]) == list(ours["first"])
-    ours_from_ref = _run(tmp_path, "load", ours_lib, model, str(tmp_path / "ref.state"), "ours_from_ref")
-    assert list(ours_from_ref["again"]) == list(ref["first"])
-    assert np.abs(ours_from_ref["logits"] - ref["logits"]).max() <= 2e-2 * np.abs(ref["logits"]).max()
+    check_state_interop(tmp_path, lib_path("pyfastllama.so"))

@@ -1,8 +1,9 @@
-"""CPU: Model.save_state / load_state through the UNCHANGED reference bridge on top of libggml_b200, with the KV cache
-living in "device" memory (the CPU stand-in of the device layer, tests/mock).  The bridge touches kv_self.{k,v}->data on
-the host without telling ggml -- except for a ggml_nbytes(k) call right before each access (reference lib/llama.cpp:57-78),
-which is the hook libggml_b200 uses to copy the cache back and to schedule its re-upload.  Checks: a state saved by us
-resumes identically in us AND in the reference library, and a state saved by the reference resumes identically in us."""
+"""CPU: Model.save_state / load_state of pyfastllama.so on top of libggml_b200, with the KV cache living in "device" memory
+(the CPU stand-in of the device layer, tests/mock).  The library touches kv_self.{k,v}->data on the host right after a
+ggml_nbytes(k) call, which is the hook libggml_b200 uses to copy the cache back and to schedule its re-upload.  Checks: a
+state saved by us resumes identically in us; it carries what the reference library writes at the same point (its state file
+and tokens are stored in tests/golden/model_state_toy.npz, oracle/gen_golden_model.py); and a state saved by the reference
+resumes in us with the reference's tokens."""
 import os
 import subprocess
 import sys
@@ -53,27 +54,64 @@ def _run(tmp_path, mode, lib, model, state, tag):
     return np.load(out)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(MOCK, "pyfastllama.so")), reason="tests/mock not built (needs the drop-in library)")
-def test_state_round_trip_and_interop_with_reference(tmp_path):
+def state_model(tmp_path):
     from fastllama_b200.ggjt import Q4_0, write_synthetic_numpy
-    from oracle.pyoracle import REF_PYFASTLLAMA_SO, Oracle
+    from oracle.pyoracle import Oracle
 
-    if not os.path.exists(REF_PYFASTLLAMA_SO):
-        pytest.skip("oracle/_ref not built")
     orc = Oracle()
     model = str(tmp_path / "toy.bin")
     write_synthetic_numpy(model, Q4_0, n_vocab=512, n_embd=256, n_mult=256, n_head=4, n_layer=3, seed=7, std=0.01, quantize=lambda w, t: orc.quantize_q4(w, t))
-    ours_lib = os.path.join(MOCK, "pyfastllama.so")
+    return model
+
+
+def parse_state(raw: bytes) -> dict:
+    """The fields of a state file: i32 n_past, u64 + text of the RNG, u64 mem_per_token, u64 + i32[] pending tokens, u64 + i32[]
+    last tokens, u64 + f32[] logits, u64 + i32[] system prompt, i32 KV type, then K and V (f32, equal halves)."""
+    out, off = {}, 0
+
+    def take(dtype, n):
+        nonlocal off
+        a = np.frombuffer(raw, dtype=dtype, count=n, offset=off)
+        off += a.nbytes
+        return a
+
+    out["n_past"] = int(take(np.int32, 1)[0])
+    out["rng"] = take(np.uint8, int(take(np.uint64, 1)[0])).tobytes()
+    out["mem_per_token"] = int(take(np.uint64, 1)[0])
+    for name, dt in (("pending", np.int32), ("last_tokens", np.int32), ("logits", np.float32), ("system_prompt", np.int32)):
+        out[name] = take(dt, int(take(np.uint64, 1)[0]))
+    out["kv_type"] = int(take(np.int32, 1)[0])
+    kv = np.frombuffer(raw, dtype=np.float32, offset=off)
+    out["k"], out["v"] = kv[: kv.size // 2], kv[kv.size // 2:]
+    return out
+
+
+def check_state_interop(tmp_path, ours_lib):
+    model = state_model(tmp_path)
+    golden = np.load(os.path.join(ROOT, "tests", "golden", "model_state_toy.npz"))
+    ref_state = tmp_path / "ref.state"
+    ref_state.write_bytes(golden["state"].tobytes())
 
     ours = _run(tmp_path, "save", ours_lib, model, str(tmp_path / "ours.state"), "ours")
     assert list(ours["first"]) == list(ours["again"])                       # our own state resumes identically in us
-    ref = _run(tmp_path, "save", REF_PYFASTLLAMA_SO, model, str(tmp_path / "ref.state"), "ref")
-    assert list(ref["first"]) == list(ref["again"])
-    assert os.path.getsize(tmp_path / "ours.state") == os.path.getsize(tmp_path / "ref.state")
+    assert list(golden["first"]) == list(golden["again"])
+    assert list(ours["first"]) == list(golden["first"])
+    assert os.path.getsize(tmp_path / "ours.state") == ref_state.stat().st_size
 
-    ref_from_ours = _run(tmp_path, "load", REF_PYFASTLLAMA_SO, model, str(tmp_path / "ours.state"), "ref_from_ours")
-    assert list(ref_from_ours["again"]) == list(ours["first"])              # the KV cache we copied back is what the reference expects
-    ours_from_ref = _run(tmp_path, "load", ours_lib, model, str(tmp_path / "ref.state"), "ours_from_ref")
-    assert list(ours_from_ref["again"]) == list(ref["first"])               # a cache loaded on the host reaches the device
-    tol = 2e-2 * np.abs(ref["logits"]).max()
-    assert np.abs(ours_from_ref["logits"] - ref["logits"]).max() <= tol
+    # what the reference would resume from: every field of our state file is the reference's, the floats within the logits' budget
+    # (mem_per_token is informational and differs: the reference's compute arena also holds its CPU work buffer)
+    a, b = parse_state((tmp_path / "ours.state").read_bytes()), parse_state(ref_state.read_bytes())
+    for key in ("n_past", "rng", "pending", "last_tokens", "system_prompt", "kv_type"):
+        assert np.array_equal(a[key], b[key]), key
+    for key in ("logits", "k", "v"):
+        assert a[key].shape == b[key].shape and np.abs(a[key] - b[key]).max() <= 2e-2 * np.abs(b[key]).max(), key
+
+    ours_from_ref = _run(tmp_path, "load", ours_lib, model, str(ref_state), "ours_from_ref")
+    assert list(ours_from_ref["again"]) == list(golden["first"])            # a cache loaded on the host reaches the device
+    tol = 2e-2 * np.abs(golden["logits"]).max()
+    assert np.abs(ours_from_ref["logits"] - golden["logits"]).max() <= tol
+
+
+@pytest.mark.skipif(not os.path.exists(os.path.join(MOCK, "pyfastllama.so")), reason="tests/mock not built (needs the drop-in library)")
+def test_state_round_trip_and_interop_with_reference(tmp_path):
+    check_state_interop(tmp_path, os.path.join(MOCK, "pyfastllama.so"))
